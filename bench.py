@@ -21,6 +21,9 @@ device.  The 1 B-pair job does not fit any memory, so it is streamed: a "step" i
   cpu_baseline  the CPU oracle (port of the reference; the Rust reference cannot be built here)
 
 `--impl reference` times that oracle on all host cores instead (rank 0 only).
+
+`--dump-outputs DIR` writes what the caller of the timed step received after its last step (rank 0) as
+DIR/<name>.npy; the inputs are the same seeded batch in every run, so two builds compare output for output.
 """
 from __future__ import annotations
 
@@ -36,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree (it may be read-only)
 
 READ_LEN = 150
 MIN_BASEQ = 20
@@ -248,7 +252,11 @@ def main():
                     help="pairs of the files+gzip leg's second, larger run of the `fasta` binary (0 = skip)")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="no device-time legs for BASELINE configs[0..3]")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, ~34 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -345,6 +353,8 @@ def main():
     if world > 1:
         assert counts[N_SAMPLES] == P * world, "all-reduced total_reads must cover every rank"
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:  # before the passes below reuse the slot's buffers
+        dump_outputs(args.dump_outputs, eng, L, res, counts)
     ms_step = ms_total / steps
     value = 2.0 * P * world / (ms_step * 1e-3)
     ms_with_compaction = ms_step
@@ -711,6 +721,48 @@ def run_add_barcode_leg(local_rank, peak, n=1_000_000):
         return {"reads": n, "ms": ms, "ms_barcode_table": ms_table, "engine_bits": int(r.reserved), "launches": int(r.gpu_launches), "algorithmic_bytes": b, "achieved": b / (ms * 1e-3) / 1e9,
                 "frac": b / (ms * 1e-3) / 1e9 / peak, "reads_per_s": n / (ms * 1e-3),
                 "workload": "fasta add barcode, 1 M reads + 1 M barcode records (i7+i5UMI on the sequence line)"}
+
+
+def dump_outputs(out_dir, eng, L, res, counts, n_sample=1 << 22, seed=2024):
+    """What the caller of the timed step receives, as DIR/<name>.npy:
+
+      counts                  float64 [S + 2]  reads per sample, then total and identified reads
+      mate{1,2}_sample_len    float64 [S]      bytes of each sample's output stream (the content of its .fq.gz file)
+      mate{1,2}_sample_crc32  float64 [S]      CRC-32 of each sample's stream, so every byte is compared
+      mate{1,2}_bytes         float32 [n]      a seeded sample of the bytes of the streams laid end to end in sheet
+                                               order (sorted positions drawn from the streams' total length)
+
+    The streams are read through the slice table: the padding between slices of the compacted buffer is not
+    output and is never read."""
+    import zlib
+    import numpy as np
+    lib, S = eng.lib, N_SAMPLES
+    arrays = {"counts": np.array(counts[:S + 2], dtype=np.float64)}
+    for m in range(2):
+        ext = int(res.out_extent[m])
+        buf = np.empty(max(ext, 1), dtype=np.uint8)
+        sl = (L.Slice * (S + 1))()
+        assert lib.sk_download_compact(eng.ctx, 0, m, buf.ctypes.data, ext) == 0, lib.sk_last_error(eng.ctx)
+        assert lib.sk_download_slices(eng.ctx, 0, m, sl) == 0, lib.sk_last_error(eng.ctx)
+        eng.wait()
+        off = np.array([sl[s].offset for s in range(S)], dtype=np.int64)
+        ln = np.array([sl[s].len for s in range(S)], dtype=np.int64)
+        assert np.all(off + ln <= ext) and int(ln.sum()) == int(res.out_bytes[m]), "slice table and outcome disagree"
+        mv = memoryview(buf)
+        arrays["mate%d_sample_len" % (m + 1)] = ln.astype(np.float64)
+        arrays["mate%d_sample_crc32" % (m + 1)] = np.array([zlib.crc32(mv[o:o + n]) for o, n in zip(off, ln)],
+                                                           dtype=np.float64)
+        total = int(ln.sum())
+        pos = np.sort(np.random.default_rng(seed + m).integers(0, max(total, 1), size=min(n_sample, total)))
+        start = np.cumsum(ln) - ln
+        s = np.searchsorted(start, pos, side="right") - 1  # the sample whose stream holds each position
+        arrays["mate%d_bytes" % (m + 1)] = buf[off[s] + pos - start[s]].astype(np.float32)
+        del buf, mv
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("bench: wrote %d arrays (%.1f MB) to %s" % (len(arrays), sum(a.nbytes for a in arrays.values()) / 1e6, out_dir),
+          file=sys.stderr)
 
 
 def verify_ranges(torch, L, bcs, local_rank, rank, world, n=1_000_000):
